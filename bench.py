@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — tasks/sec of the task fan-out hot path on N B200s (contract: DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 1|2|3|4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 1|2|3|4] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch: every pending task of the batch is popped,
@@ -9,9 +9,10 @@ deserialised, run through the handler and serialised (one persistent drain kerne
 Default workload = BASELINE.json configs[1]: 1M x 256-character identity tasks per GPU (weak scaling:
 every rank owns its own shard of the pending ring; no data-path collective in the drain).
 
-  value        whole-job tasks/s, batch resident in HBM: the MEDIAN of B bursts of exactly K steps each (B is chosen
-               so that the timed bursts add up to >= --sustain-seconds); every burst is bracketed by a barrier and a
-               synchronise on both sides and timed with CUDA events on the drain stream, max over ranks
+  value        whole-job tasks/s, batch resident in HBM: W untimed steps, then ONE burst of exactly K timed steps,
+               bracketed by a barrier and a synchronise on both sides and timed with CUDA events on the drain stream,
+               max over ranks (--sustain-seconds S > 0 repeats the burst until the timed bursts add up to S and takes
+               the median burst)
   e2e          the same through the C ABI with HOST buffers: b9_batch_push_async (H2D from pinned memory) + b9_drain (D2H)
   e2e_packed   the same starting from payloads scattered over PAGEABLE memory: b9_batch_push_v (the pack step) + b9_drain
   link         what the host<->device link gives on this box for the e2e byte counts (all ranks at once): e2e's roofline
@@ -19,6 +20,10 @@ every rank owns its own shard of the pending ring; no data-path collective in th
   rebalance    N > 1: skewed ingest (rank 0 holds 2x its share), ONE b9_rebalance (NCCL all-to-all), then the drain
   cpu_baseline the oracle's C port of the reference loop on this box's host cores (rank 0, N = 1), plus the 1-thread rate
                and BASELINE.md's C1 (the Python loop, one process, configs[0])
+
+--dump-outputs DIR writes the records the last timed step handed back (rank 0; with --impl reference, the C port's)
+as DIR/<name>.npy, see dump_outputs(). The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -58,11 +63,13 @@ def parse_args():
     ap.add_argument("--chars", type=int, default=256)
     ap.add_argument("--handler", default="", help="override the config's handler")
     ap.add_argument("--e2e-steps", type=int, default=120, help="steps of the end-to-end legs (about a second of timed region at one GPU)")
-    ap.add_argument("--sustain-seconds", type=float, default=1.0, help="bursts of K steps are repeated until their timed regions add up to this")
+    ap.add_argument("--sustain-seconds", type=float, default=0.0,
+                    help="0: one burst of K timed steps; S > 0: bursts of K steps are repeated until their timed regions add up to S")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cancelled", type=float, default=0.0, help="fraction of the resident tasks pushed with B9_TF_CANCELLED")
     ap.add_argument("--skew", type=float, default=1.0, help="N>1 rebalance leg: rank 0 ingests (1+skew)x its fair share; 0 = no rebalance leg")
     ap.add_argument("--adversarial", type=float, default=0.01, help="share of tasks whose string needs escaping (SURVEY.md §8d: 1 %%)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR", help="write the last timed step's records to DIR/<name>.npy")
     a = ap.parse_args()
     h, total, g = CONFIGS[a.config]
     if not a.handler:
@@ -239,6 +246,33 @@ def workload_name(args, n) -> str:
     return f"configs[{args.config}]: {args.handler}, {n} tasks per GPU"
 
 
+DUMP_SEED = 20261017
+DUMP_RECORDS = 1 << 15
+DUMP_LIMIT_BYTES = 60_000_000        # the data of all files; their headers add well under a kilobyte
+
+
+def dump_outputs(out_dir, task_ids, status, has_result, starts, lengths, blob) -> None:
+    """--dump-outputs: records of one step, in record (= task) order, as .npy files in out_dir. A fixed, seeded sample of
+    DUMP_RECORDS records (fewer when their result bytes would take the files past DUMP_LIMIT_BYTES):
+      record_index [k] float64, task_ids [k, 16], status [k], has_result [k], lengths [k]   float32
+      result_bytes [sum of lengths] float32: the sampled records' result bytes one after the other
+    Record i's bytes are blob[starts[i] : starts[i] + lengths[i]]. Where they sit in the device's blob follows the order in
+    which tiles finished, so those offsets are not written: only what they point at."""
+    n = int(status.shape[0])
+    idx = np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_RECORDS), replace=False)      # in random order
+    keep = int(np.searchsorted(np.cumsum(8 + 4 * (16 + 3) + 4 * lengths[idx].astype(np.int64)), DUMP_LIMIT_BYTES, side="right"))
+    idx = np.sort(idx[:keep])
+    ln = lengths[idx].astype(np.int64)
+    ends = np.cumsum(ln)
+    rec = np.repeat(np.arange(keep, dtype=np.int64), ln)
+    src = np.asarray(starts, dtype=np.int64)[idx][rec] + (np.arange(int(ends[-1]) if keep else 0, dtype=np.int64) - (ends - ln)[rec])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("record_index", idx.astype(np.float64)), ("task_ids", np.asarray(task_ids)[idx].astype(np.float32)),
+                    ("status", status[idx].astype(np.float32)), ("has_result", has_result[idx].astype(np.float32)),
+                    ("lengths", ln.astype(np.float32)), ("result_bytes", blob[src].astype(np.float32))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_reference(args):
     """--impl reference: the reference's CPU task loop on this box's host cores. The Go gateway and
     the Python runner cannot be built/imported here (no Go toolchain, SDK deps missing), so this is
@@ -253,11 +287,13 @@ def run_reference(args):
     times = []
     for s in range(args.warmup + args.steps):
         t0 = time.perf_counter()
-        coracle.run_batch(batch.task_ids, batch.payload, batch.offsets, args.handler, nthreads=cores,
-                          out_cap=int(batch.payload.size) + 64)
+        o = coracle.run_batch(batch.task_ids, batch.payload, batch.offsets, args.handler, nthreads=cores,
+                              out_cap=int(batch.payload.size) + 64)
         dt = time.perf_counter() - t0
         if s >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, batch.task_ids, o.status, o.has, o.offsets[:-1], np.diff(o.offsets), o.payload)
     total = sum(times)
     v = batch.n * len(times) / total
     # the same loop on ONE thread (a bounded sample): what the port does per core, and how it scales
@@ -382,9 +418,10 @@ def main():
     launches0 = dq.stats().kernel_launches
     barrier()
     sampler.start()
-    # bursts of EXACTLY K steps: the K launches are enqueued back to back (B9_DRAIN_ASYNC), as a host that pipelines its
+    # a burst of EXACTLY K steps: the K launches are enqueued back to back (B9_DRAIN_ASYNC), as a host that pipelines its
     # drains would; a barrier + synchronise brackets every burst; the device time of a burst comes from CUDA events on
-    # the drain stream (first step's start -> last step's end), the max over ranks is the burst's time
+    # the drain stream (first step's start -> last step's end), the max over ranks is the burst's time. One burst unless
+    # --sustain-seconds asks for more.
     burst_dev, burst_wall = [], []
     timed_total = 0.0
     launches_per_burst = None
@@ -407,14 +444,14 @@ def main():
             break
     clocks = sampler.stop()
     launches = dq.stats().kernel_launches - launches0
+    if args.dump_outputs and rank == 0:
+        last = dq.fetch()                            # the last timed step's records (peek: the batch stays resident)
+        dump_outputs(args.dump_outputs, last.task_ids, last.status, last.has_result, last.offsets, last.lengths, last.payload)
+        del last
     elapsed = statistics.median(burst_dev)
     wall_elapsed = statistics.median(burst_wall)
     value = n_total * args.steps / elapsed
-    kernel_ms = []
-    for _ in range(5):                               # per-step kernel time (CUDA events around one step's kernel), outside the bursts
-        dq.drain_launch(args.handler, n, peek=True)
-        kernel_ms.append(dq.stats().last_drain_kernel_ms)
-    k_ms = reduce_max(statistics.mean(kernel_ms))
+    k_ms = 1e3 * elapsed / args.steps                # device time per timed step (back to back: the gaps between launches count)
     # drop the resident batch; its records are the reference records of the legs below
     dq.drain_launch(args.handler, n, peek=False)
     res = dq.fetch()
@@ -618,11 +655,12 @@ def main():
         line = {
             "metric": "tasks_per_sec", "value": value, "unit": "tasks/s", "n_gpus": world, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1e3 * elapsed / args.steps, "wall_ms_per_step": 1e3 * wall_elapsed / args.steps,
-            "timing": {"bursts": len(burst_dev), "steps_per_burst": args.steps, "timed_seconds": timed_total,
+            "timing": {"bursts": len(burst_dev), "steps_per_burst": args.steps, "timed_steps": len(burst_dev) * args.steps,
+                       "timed_seconds": timed_total,
                        "burst_ms_min_median_max": [1e3 * min(burst_dev), 1e3 * elapsed, 1e3 * max(burst_dev)],
                        "how": "every burst = exactly K steps enqueued back to back (B9_DRAIN_ASYNC), CUDA events on the drain stream, "
-                              "barrier + synchronise on both sides, max over ranks; value uses the median burst; wall_ms_per_step = "
-                              "host clock over the median burst, barriers included"},
+                              "barrier + synchronise on both sides, max over ranks; one burst unless --sustain-seconds > 0, then value "
+                              "uses the median burst; wall_ms_per_step = host clock over the median burst, barriers included"},
             "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "u8" if args.handler != "vadd_f32" else "f32", "data": "synthetic",
             "config": {"workload": workload_name(args, n) + ", resident in HBM",
@@ -632,7 +670,8 @@ def main():
                        "l2": f"inputs {in_bytes / 1e6:.0f} MB + outputs {out_bytes / 1e6:.0f} MB per step exceed the 126 MB L2; no flush needed"},
             "roofline": {"bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak,
                          "traffic": traffic, "traffic_source": traffic_src, "kernel": f"b9::drain3_kernel<{args.handler}>",
-                         "kernel_ms": k_ms, "algorithmic_bytes_per_task": algo / n, "peak_source": peak_src},
+                         "kernel_ms": k_ms, "kernel_ms_how": "device time of the median burst / K",
+                         "algorithmic_bytes_per_task": algo / n, "peak_source": peak_src},
             "cpu_baseline": cpu,
             "e2e": {"value": e2e_value, "unit": "tasks/s", "h2d_bytes_per_step": int(h2d), "d2h_bytes_per_step": int(d2h),
                     "steps": args.e2e_steps, "ms_per_step": 1e3 * e2e_elapsed / args.e2e_steps,

@@ -189,11 +189,10 @@ def main():
     print(path, n, "task executions through the reference runner")
 
 
-def fuzz(n_payloads: int, seed: int) -> int:
-    """Live check (no files written): random SDK-style payloads -> the oracle's wire records -> the
-    reference runner; every status / result must equal the oracle's. Returns the number of mismatches."""
+def fuzz_payloads(n_payloads: int, seed: int):
+    """-> (payloads, task ids): random SDK-style put payloads, the same ones for the same (n_payloads, seed)."""
     import random
-    rt, rc = load_reference_runner()
+    sys.path.insert(0, ROOT)
     from oracle.pyoracle import loop
     rnd = random.Random(seed)
     alphabet = ["a", "Z", "0", " ", '"', "\\", "/", "<", ">", "&", "\n", "\t", "\x01", "\x7f", "\u00e9", "\u2028", "\u20ac",
@@ -223,7 +222,15 @@ def fuzz(n_payloads: int, seed: int) -> int:
         elif shape == 3: args, kwargs = tuple(rval() for _ in range(rnd.randint(0, 3))), {}
         else: args, kwargs = tuple(rval() for _ in range(rnd.randint(0, 2))), {rstr(): rval() for _ in range(rnd.randint(0, 2))}
         payloads.append(loop.sdk_put_payload(*args, **kwargs))
-    ids = [rnd.randbytes(16) for _ in payloads]
+    return payloads, [rnd.randbytes(16) for _ in payloads]
+
+
+def fuzz(n_payloads: int, seed: int) -> int:
+    """Live check (no files written): random SDK-style payloads -> the oracle's wire records -> the
+    reference runner; every status / result must equal the oracle's. Returns the number of mismatches."""
+    rt, rc = load_reference_runner()
+    from oracle.pyoracle import loop
+    payloads, ids = fuzz_payloads(n_payloads, seed)
     bad = 0
     for h in HANDLERS:
         want = loop.run_task_loop(payloads, ids, h, keep_wire=True)
@@ -238,7 +245,47 @@ def fuzz(n_payloads: int, seed: int) -> int:
     return bad
 
 
+def fuzz_digest(payloads, ids) -> str:
+    import hashlib
+    h = hashlib.sha256()
+    for p, i in zip(payloads, ids):
+        h.update(i); h.update(len(p).to_bytes(8, "little")); h.update(p)
+    return h.hexdigest()
+
+
+def freeze_fuzz(n_payloads: int, seed: int) -> None:
+    """What the reference runner completed the wire records of fuzz_payloads(n_payloads, seed) with ->
+    tests/golden/ref_runner_fuzz_golden.json.gz, which tests/test_oracle_vs_ref_runner.py compares the oracle with.
+    The payloads themselves are regenerated from the seed; their digest is stored to catch a changed generator."""
+    import gzip
+    rt, rc = load_reference_runner()
+    from oracle.pyoracle import loop
+    payloads, ids = fuzz_payloads(n_payloads, seed)
+    out = {"source": "reference runner loop (sdk/src/beta9/runner/taskqueue.py:297-404) over the oracle's wire records",
+           "n_payloads": n_payloads, "seed": seed, "payloads_sha256": fuzz_digest(payloads, ids), "handlers": {}}
+    for h in HANDLERS:
+        live = loop.run_task_loop(payloads, ids, h, keep_wire=True)
+        done = iter(run_reference_worker(rt, rc, h, [w.wire for w in live if w.wire is not None]))
+        # one entry per payload: None where put refused it (no task, no runner), else what the runner completed it with
+        per = []
+        for w in live:
+            if w.wire is None:
+                per.append(None)
+                continue
+            _, status, result = next(done)
+            per.append([str(status), None if result is None else base64.b64encode(result).decode()])
+        assert next(done, None) is None
+        out["handlers"][h] = per
+    path = os.path.join(ROOT, "tests", "golden", "ref_runner_fuzz_golden.json.gz")
+    with gzip.GzipFile(path, "wb", mtime=0) as f:
+        f.write(json.dumps(out, sort_keys=True).encode())
+    print(path, n_payloads, "payloads x", len(HANDLERS), "handlers through the reference runner")
+
+
 if __name__ == "__main__":
     if len(sys.argv) >= 3 and sys.argv[1] == "--fuzz":
         sys.exit(1 if fuzz(int(sys.argv[2]), int(sys.argv[3]) if len(sys.argv) > 3 else 0xB9) else 0)
+    if len(sys.argv) >= 3 and sys.argv[1] == "--freeze-fuzz":
+        freeze_fuzz(int(sys.argv[2]), int(sys.argv[3]) if len(sys.argv) > 3 else 0xB9)
+        sys.exit(0)
     main()

@@ -60,13 +60,21 @@ def test_scale_func_known_answers_through_abi(so_path, q, tpc, mc, mr, desired, 
 
 
 def test_no_device_fails_loudly(so_path):
-    lib = L.load()
-    if lib.b9_device_count() > 0:
-        pytest.skip("a GPU is present")
-    from beta9_b200.device_queue import DeviceQueue
-    with pytest.raises(L.B9Error) as e:
-        DeviceQueue()
-    assert e.value.code == L.B9_ENODEV and "no CPU path" in str(e.value)
+    """In a process that sees no CUDA device (CUDA_VISIBLE_DEVICES="" hides those of a GPU machine), creating a
+    queue raises B9_ENODEV with the "no CPU path" message."""
+    import sys
+    code = ("from beta9_b200 import _lib as L\n"
+            "from beta9_b200.device_queue import DeviceQueue\n"
+            "assert L.load().b9_device_count() == 0\n"
+            "try:\n"
+            "    DeviceQueue()\n"
+            "except L.B9Error as e:\n"
+            "    assert e.code == L.B9_ENODEV and 'no CPU path' in str(e), (e.code, str(e))\n"
+            "else:\n"
+            "    raise AssertionError('DeviceQueue() without a device did not raise')\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, capture_output=True, text=True, timeout=120,
+                       env={**os.environ, "CUDA_VISIBLE_DEVICES": ""})
+    assert r.returncode == 0, r.stderr[-2000:]
 
 
 def test_header_is_plain_c99_and_the_c_example_links(so_path, tmp_path):

@@ -81,14 +81,26 @@ def test_map_input_formatting_equals_the_reference_sdks(goldens):
         assert _CallableWrapper._format_args(x) == case["out"], case
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/sdk/src"), reason="the reference checkout is not mounted here")
 def test_live_fuzz_against_the_reference_runner():
-    """Where /root/reference exists (this container, not the GPU box): 1200 random SDK-style payloads
-    x 4 handlers through the reference's runner loop, in a subprocess (the harness sets a runner
-    container's environment variables), every completion compared with the oracle."""
-    import subprocess
-    import sys
-    r = subprocess.run([sys.executable, os.path.join(HERE, "golden", "make_ref_runner_golden.py"), "--fuzz", "1200", "20260921"],
-                       capture_output=True, text=True, timeout=600, cwd=os.path.dirname(HERE))
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]
-    assert "0 mismatches" in r.stdout
+    """1200 random SDK-style payloads x 4 handlers through the oracle, every completion compared with what the
+    reference's runner loop completed the same wire records with (tests/golden/ref_runner_fuzz_golden.json.gz,
+    written by make_ref_runner_golden.py --freeze-fuzz 1200 20260921)."""
+    import gzip
+    from tests.golden.make_ref_runner_golden import fuzz_digest, fuzz_payloads
+    with gzip.open(os.path.join(HERE, "golden", "ref_runner_fuzz_golden.json.gz")) as f:
+        ref = json.load(f)
+    payloads, ids = fuzz_payloads(ref["n_payloads"], ref["seed"])
+    assert fuzz_digest(payloads, ids) == ref["payloads_sha256"]           # the payloads the reference runner saw
+    assert sorted(ref["handlers"]) == sorted(HANDLERS)
+    bad = []
+    for h in HANDLERS:
+        live = loop.run_task_loop(payloads, ids, h, keep_wire=True)
+        assert len(live) == len(ref["handlers"][h])
+        for i, (w, r) in enumerate(zip(live, ref["handlers"][h])):
+            if r is None:                                                   # refused at put: no runner involved
+                assert w.wire is None, (h, i)
+                continue
+            want = None if r[1] is None else base64.b64decode(r[1])
+            if w.wire is None or w.status != r[0] or w.result != want:
+                bad.append((h, i, payloads[i][:80], (w.status, w.result), (r[0], want)))
+    assert not bad, bad[:5]
