@@ -703,7 +703,10 @@ __device__ __forceinline__ int json_sum_coop(const uint8_t* __restrict__ p, uint
     ve = __reduce_min_sync(0xffffffffu, ve);
 
     // ---- 4b. Horner over the numbers that START in my chunk (a number cut by the chunk end is finished from
-    // the next chunk's words); no data-dependent branch: run ends, the span and my head digits are masks
+    // the next chunk's words); no data-dependent branch: run ends, the span and my head digits are masks.
+    // No overflow check: a document of <= JSON_COOP_MAX_DOC = 4096 bytes spends 11 on `{"values":[` and 2 on `]}`; a
+    // value of d <= 15 digits (< 10^d) takes d + 1 bytes with its ',', so 15-digit ones add the most per byte; k of them
+    // take 16k - 1 <= 4083 bytes, k <= 255: sum < 255 * 10^15 ~ 2.6e17, far below 2^63 ~ 9.2e18 (values are >= 0 here).
     unsigned long long sum = 0;
     for (uint32_t seg = 0; seg < nseg; ++seg) {
         const uint32_t base = (seg << 10) + 32u * (uint32_t)lane;

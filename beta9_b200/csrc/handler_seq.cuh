@@ -120,7 +120,8 @@ __device__ inline void handler_phase_a(int handler, const uint8_t* __restrict__ 
         if (st) { rec.status = (uint8_t)st; return; }
         if (sum == 0) return;
         rec.value = sum; rec.mode = OM_I64_DEC; rec.has = 1;
-        rec.out_len = dec_len_u64((unsigned long long)(sum < 0 ? -sum : sum)) + (sum < 0 ? 1u : 0u);
+        const unsigned long long mag = sum < 0 ? 0ull - (unsigned long long)sum : (unsigned long long)sum;   // (INT64_MIN too)
+        rec.out_len = dec_len_u64(mag) + (sum < 0 ? 1u : 0u);
         return;
     }
     default:
@@ -132,9 +133,9 @@ __device__ inline void handler_phase_a(int handler, const uint8_t* __restrict__ 
 __device__ inline void seq_emit(const uint8_t* __restrict__ p, const TaskRec& rec, uint8_t* __restrict__ o) {
     if (rec.mode == OM_VADD) vadd_write(p, rec.src_off, rec.src_len, o);
     else if (rec.mode == OM_U32_DEC || rec.mode == OM_I64_DEC) {
-        long long v = rec.value; uint32_t l = rec.out_len;
-        if (v < 0) { *o++ = '-'; --l; v = -v; }
-        write_dec(o, (unsigned long long)v, l);
+        unsigned long long v = (unsigned long long)rec.value; uint32_t l = rec.out_len;
+        if (rec.value < 0) { *o++ = '-'; --l; v = 0ull - v; }          // magnitude without a signed negation (INT64_MIN)
+        write_dec(o, v, l);
     } else if (rec.mode == OM_STR_ESC) {                          // string the sequential parser sized (non-canonical frame)
         uint32_t i = rec.src_off + 1, end = rec.src_off + rec.src_len - 1;
         *o++ = '"';

@@ -50,7 +50,8 @@ __device__ inline uint32_t crc32_of_string_token(const uint8_t* __restrict__ p, 
 }
 
 // ---------------------------------------------------------------- json_sum (sum(obj["values"]))
-// status: 0 ok (value in *sum), 1 ERROR (KeyError / TypeError), 4 UNSUPPORTED (a float in the list)
+// status: 0 ok (value in *sum), 1 ERROR (KeyError / TypeError), 4 UNSUPPORTED (a float in the list, or a partial
+// sum outside int64: Python's int is exact there, and the host's CPU loop answers)
 __device__ inline bool key_is_values(const uint8_t* __restrict__ p, uint32_t s, uint32_t e) {
     const char V[] = "values";
     uint32_t k = 0, i = s;
@@ -81,10 +82,12 @@ __device__ inline int sum_values_token(const uint8_t* __restrict__ p, uint32_t v
             if (simple) {
                 bool neg = d == '-'; long long v = 0;
                 for (uint32_t k = i + (neg ? 1 : 0); k < (uint32_t)e; ++k) v = v * 10 + (p[k] - '0');
-                acc += neg ? -v : v;
+                const long long s = neg ? -v : v;                   // |s| < 10^15: only the add can leave int64
+                if (s > 0 ? acc > INT64_MAX - s : acc < INT64_MIN - s) unsupported = true;
+                else acc += s;
             } else unsupported = true;                              // needs float64 arithmetic / repr
             i = (uint32_t)e;
-        } else if (d == 't') { acc += 1; i += 4; }                 // True + 1 == 2
+        } else if (d == 't') { if (acc == INT64_MAX) unsupported = true; else acc += 1; i += 4; }   // True + 1 == 2
         else if (d == 'f') { i += 5; }
         else return 1;                                             // None / str / list / dict: TypeError
         while (i < ve && is_ws(p[i])) ++i;

@@ -666,7 +666,8 @@ static int run_handler(int h, val_t *args, val_t *kwargs, buf_t *out, int *has, 
             acc += (__int128)strtoll((const char *)x->lit, NULL, 10);  /* literal is followed by , or ] */
         }
         if (any_float) return B9O_UNSUPPORTED;
-        if (acc > ((__int128)1 << 62) || acc < -((__int128)1 << 62)) return B9O_UNSUPPORTED;
+        /* Python's sum is exact; this prints int64. The device decides nothing outside int64 either. */
+        if (acc > (__int128)INT64_MAX || acc < (__int128)INT64_MIN) return B9O_UNSUPPORTED;
         if (acc == 0) return B9O_COMPLETE;
         char t[32]; int l = snprintf(t, sizeof t, "%lld", (long long)acc); buf_put(out, t, (size_t)l);
         *has = 1; return B9O_COMPLETE;

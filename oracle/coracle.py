@@ -47,7 +47,8 @@ def lib() -> ctypes.CDLL:
 
 
 class OracleResult:
-    def __init__(self, status, has, offsets, payload, wire_offsets=None, wire=None):
+    def __init__(self, status, has, offsets, payload, wire_offsets=None, wire=None, handler=None):
+        self.handler = handler        # the handler name the batch ran
         self.status = status          # uint8 [n]
         self.has = has                # uint8 [n]
         self.offsets = offsets        # uint64 [n+1]
@@ -93,7 +94,7 @@ def run_batch(task_ids: np.ndarray, payload: np.ndarray, offsets: np.ndarray, ha
         raise MemoryError("oracle output capacity too small")
     if keep_wire:
         w = w[:int(w_off[-1])]
-    return OracleResult(status, has, out_off, out[:total], w_off, w)
+    return OracleResult(status, has, out_off, out[:total], w_off, w, handler)
 
 
 def task_queue_scale(q: int, tpc: int, max_containers: int, max_replicas: int) -> Tuple[int, bool]:

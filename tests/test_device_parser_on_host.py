@@ -22,6 +22,12 @@ GXX = os.environ.get("CXX", "g++")
 
 @pytest.fixture(scope="module")
 def parser():
+    return load_host_shim()
+
+
+def load_host_shim():
+    """Builds (when a source is newer) and loads the host shim; returns parse(b, http) with .run, .transcode, .rfc3339
+    and .vadd_fast attached. Skips the calling test where there is no host C++ compiler."""
     csrc = os.path.join(os.path.dirname(HERE), "beta9_b200", "csrc")
     deps = [os.path.join(csrc, f) for f in os.listdir(csrc) if f.endswith((".cuh", ".h"))]
     if not os.path.exists(SO) or os.path.getmtime(SO) < max([os.path.getmtime(SRC)] + [os.path.getmtime(d) for d in deps]):

@@ -82,6 +82,25 @@ def test_json_sum():
     compare(synth.json_batch(100, doc_bytes=300, seed=2), "identity")
 
 
+def test_json_sum_near_the_int64_limits():
+    """Sums of |s| in (2^62, 2^64) in both signs, of random values below 2^53 (exact in float64): the C oracle prints
+    every sum inside int64 exactly as Python does, and declines only the ones outside."""
+    rng = random.Random(62)
+    totals = [2**62 + 1, 2**63 - 2, 2**63 - 1, 2**63, 2**63 + 1, 2**64 - 1] + [rng.randrange(2**62, 2**63) for _ in range(20)]
+    payloads, outside = [], 0
+    for t in totals + [-t for t in totals]:
+        vals, left = [], t
+        while abs(left) > 2**53:
+            v = rng.randrange(2**52, 2**53) * (1 if left > 0 else -1)
+            vals.append(v)
+            left -= v
+        vals.append(left)
+        rng.shuffle(vals)
+        payloads.append(loop.sdk_put_payload({"values": vals}))
+        outside += not -2**63 <= t < 2**63
+    assert compare(synth.from_payloads(payloads), "json_sum", allow_unsupported=True) == outside
+
+
 HANDCRAFTED = [
     b'{"args": ["x"], "kwargs": {}}', b'{"args":["x"]}', b' { "kwargs" : { } , "args" : [ "x" ] } ',
     b'{"args": [""], "kwargs": {}}', b'{"args": [], "kwargs": {}}', b'{"args": ["a", "b"], "kwargs": {}}',
@@ -107,6 +126,11 @@ HANDCRAFTED = [
     # overwrites it (decode.go keeps the first conversion error); under an unknown key it is never converted
     b'{"args": [1e999], "args": ["x"]}', b'{"args": [{"k": 5e08858}], "\\u0061rgs": []}', b'{"kwargs": {"a": 1e999, "a": 1}, "args": ["x"]}',
     b'{"args": ["x"], "kwargs": {"a": 1e999}, "kwargs": {"a": 2}}', b'{"args": ["x"], "other": 1e999, "other": 1}', b'{"args": 1e999, "args": ["x"]}',
+    # json_sum at -2^63, 2^63 - 1 (the int64 limits: decided, printed exactly) and 2^63 (beyond: the C oracle declines)
+    # as sums of 2^53 = 9007199254740992, the largest power of two whose neighbours float64 still holds exactly
+    b'{"args": [{"values": [' + b", ".join([b"-9007199254740992"] * 1024) + b']}], "kwargs": {}}',
+    b'{"args": [{"values": [' + b", ".join([b"9007199254740992"] * 1023 + [b"9007199254740991"]) + b']}], "kwargs": {}}',
+    b'{"args": [{"values": [' + b", ".join([b"9007199254740992"] * 1024) + b']}], "kwargs": {}}',
 ]
 
 
